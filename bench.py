@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference --steps K --warmup W    (the CPU arm: oracle port on the host cores)
+  python bench.py ... --dump-outputs DIR                   (also writes the last timed step's output to DIR/*.npy)
 
 Workload (BASELINE.json metric): Wan2.2-T2V-14B architecture (D 5120, 40 heads, ffn 13824, 40 layers), 720p x 81f
 latent 16x21x90x160 -> 75 600 tokens, Video-Sparse attention at sparsity 0.9 (top-k 144 of 1440 tiles), synthetic
@@ -480,6 +481,8 @@ def run_gpu_arm(args, rank, world, device):
 
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"noise_pred": out})
     peaks = measured_peaks()
     peak_tf = (peaks or {}).get("bf16_tflops_sustained", 1400.0)
     peak_src = "MEASURED_PEAKS.json bf16_tflops_sustained (kernel timed inside a long step)" if peaks else "fallback 1.4 PFLOP/s sustained (B200_PROFILING.md)"
@@ -576,6 +579,15 @@ def emit(line: dict) -> None:
     out.flush()
 
 
+def dump_outputs(directory: str, arrays: dict) -> None:
+    """Writes each tensor as `directory/<name>.npy` in float32, whole: the seeded inputs make two builds of the project
+    comparable output for output (the 14B workload's prediction is 4.8 M values, 19 MB)."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def main():
     _claim_stdout()
     ap = argparse.ArgumentParser()
@@ -587,7 +599,13 @@ def main():
     ap.add_argument("--layers", type=int, default=0, help="development only: truncate the model (result is flagged)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-sizes", default="", help="CPU arm: comma-separated token counts of the block samples")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="GPU arm: write the noise prediction of the last timed step to DIR/noise_pred.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs the GPU arm (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":

@@ -1,9 +1,13 @@
 """CPU: the bench.py contract on the one arm that runs without a GPU -- `--impl reference` (the reference's CPU block, or its
-oracle port, timed on the host cores) must put exactly ONE JSON line on stdout with the keys the driver reads."""
+oracle port, timed on the host cores) must put exactly ONE JSON line on stdout with the keys the driver reads.
+GPU (last test): the GPU arm's --steps and --dump-outputs on a one-layer model."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 from conftest import ROOT
 
@@ -64,3 +68,42 @@ def test_row_family_byte_models_accept_both_forward_call_shapes():
     oc = torch.zeros(1, H, nblk, d, dtype=torch.bfloat16)
     assert bench.combine_bytes(q, oc, q, row_block=None, out=None, out_segments=(None, 64, (1, 2, 3))) == 3 * q.numel() * 2 + oc.numel() * 2
     assert bench.combine_bytes(q, oc, None) == 2 * q.numel() * 2 + oc.numel() * 2
+
+
+def test_bad_step_counts_and_a_dump_from_the_cpu_arm_are_refused():
+    for extra in (["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True,
+                           timeout=300, cwd=ROOT)
+        assert p.returncode == 2 and p.stdout.strip() == "", (extra, p.stderr[-500:])
+
+
+def test_dump_outputs_writes_float32_npy(tmp_path):
+    import torch
+    import bench
+    x = torch.randn(2, 3, 5).bfloat16()
+    bench.dump_outputs(str(tmp_path / "d"), {"noise_pred": x})
+    y = np.load(tmp_path / "d" / "noise_pred.npy")
+    assert y.dtype == np.float32 and np.array_equal(y, x.float().numpy())
+
+
+@pytest.mark.gpu
+def test_gpu_arm_steps_set_the_timed_steps_and_the_dump_is_reproducible(tmp_path):
+    """Two runs with the same seeded inputs and different --steps: the timed region launches `steps` forwards (launch count
+    scales exactly) and the two dumps agree as two bf16 roundings of the same values (separate processes are not
+    guaranteed to be bit-equal)."""
+    import torch
+    from util import assert_two_bf16_paths_close
+    lines, dumps = {}, {}
+    for steps in (1, 2):
+        d = tmp_path / f"steps{steps}"
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", str(steps), "--warmup", "1",
+                            "--layers", "1", "--no-cpu-baseline", "--dump-outputs", str(d)],
+                           capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert p.returncode == 0, p.stderr[-3000:]
+        lines[steps] = json.loads(p.stdout.strip().splitlines()[-1])
+        dumps[steps] = np.load(d / "noise_pred.npy")
+    assert lines[1]["steps"] == 1 and lines[2]["steps"] == 2
+    assert lines[1]["gpu_launches"] > 0 and lines[2]["gpu_launches"] == 2 * lines[1]["gpu_launches"]
+    y = dumps[1]
+    assert y.dtype == np.float32 and y.shape == (1, *lines[1]["config"]["latent"]) and np.isfinite(y).all()
+    assert_two_bf16_paths_close(torch.from_numpy(dumps[2]), torch.from_numpy(y), name="noise_pred, --steps 2 vs 1")

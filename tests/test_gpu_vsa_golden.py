@@ -129,24 +129,23 @@ def test_topk_kernel_against_triton_on_tie_and_nonconvergence_stress_rows():
 
 
 def test_k1_head_to_head_when_the_reference_kernel_is_present():
-    """Live side-by-side with the reference's sm_100a kernel (oracle/_ref/k1_ref.so, built from the reference sources
-    where they lie; travels with the snapshot, absent from the history). Skipped when it did not travel."""
-    from oracle.gen_golden_gpu import load_k1
+    """Side by side with the reference's sm_100a kernel K1: its output and LSE on the reference's own block lists, as
+    oracle/gen_golden_gpu.py stored them in the fixtures (ragged and full grids, the 720p one on its sampled q blocks)."""
     from fastvideo_b200 import ops
-    k1 = load_k1()
-    if k1 is None:
-        pytest.skip("oracle/_ref/k1_ref.so not present / not loadable")
-    shape, H = (9, 13, 10), 4
-    q, k, v, _, vbs, valid = padded_inputs(shape, H, seed=5, flavour="local")
-    nblk = vbs.numel()
-    qd, kd, vd, vbsd = (t.cuda() for t in (q, k, v, vbs))
-    torch.manual_seed(1)
-    keep = torch.zeros(1, H, nblk, nblk, dtype=torch.bool, device="cuda")
-    keep.scatter_(-1, torch.randn(1, H, nblk, nblk, device="cuda").topk(9, dim=-1).indices, True)
-    idx, num = ops.map_to_index(keep)
-    o1, lse1 = k1.fwd(qd, kd, vd, None, idx, num, vbsd, 128 ** -0.5, True)[:2]
-    o, lse = ops.attention_blocklist(qd.transpose(1, 2), kd.transpose(1, 2), vd.transpose(1, 2), idx, num, kv_len=vbsd,
-                                     q_len=vbsd, return_lse=True)
-    vr = valid.cuda()
-    assert (o.transpose(1, 2)[:, :, vr].float() - o1[:, :, vr].float()).abs().max().item() < OUT_ABS
-    assert (lse[:, :, vr] - lse1.reshape(lse.shape)[:, :, vr]).abs().max().item() < LSE_ABS
+    cases = [fx for name in ("vsa_gpu_small.pt", "vsa_gpu_720p.pt") for fx in _load(name).values() if "k1_out" in fx]
+    assert len(cases) >= 4
+    for fx in cases:
+        q, k, v, _, vbs, valid = padded_inputs(tuple(fx["shape"]), fx["heads"], fx["seed"], fx["flavour"])
+        nblk = vbs.numel()
+        mask = fx["mask"] if "mask" in fx else _unpack_mask(fx["mask_packed"], nblk)
+        blocks = fx.get("blocks", torch.arange(nblk))
+        rows = (blocks[:, None] * 64 + torch.arange(64)[None, :]).reshape(-1)
+        vr = valid[rows]
+        vbsd = vbs.cuda()
+        idx, num = ops.map_to_index(mask.cuda())
+        o, lse = ops.attention_blocklist(*(t.cuda().transpose(1, 2) for t in (q, k, v)), idx, num, kv_len=vbsd, q_len=vbsd,
+                                         return_lse=True)
+        o = o.transpose(1, 2).cpu()[:, :, rows][:, :, vr]
+        lse = lse.cpu()[:, :, rows][:, :, vr]
+        assert (o.float() - fx["k1_out"][:, :, vr].float()).abs().max().item() < OUT_ABS, fx["shape"]
+        assert (lse - fx["k1_lse"].reshape(lse.shape[:2] + vr.shape)[:, :, vr]).abs().max().item() < LSE_ABS, fx["shape"]

@@ -61,10 +61,11 @@ def _worker(rank, world, port, q):
         y = vae_tiling.decode(z, fake_tile_decode, cfg, rank=rank, world=world)
         # same tiles, same blend order, fp32 staging as in the reference's parallel path: equals the one-rank parallel path
         y1 = vae_tiling.parallel_tiled_decode(z, fake_tile_decode, cfg, 0, 1)[:, :, :17]
-        ok = torch.equal(y, y1) and y.dtype == torch.float32
         # and for fp32 data the parallel result equals the serial temporal+spatial tiling
         ys = vae_tiling.decode(z, fake_tile_decode, vae_tiling.TilingConfig(use_parallel_tiling=False))
-        q.put((rank, "ok" if ok and torch.equal(y, ys) else "MISMATCH"))
+        bad = [f"{int((y != r).sum())} of {y.numel()} values differ from the {n} result"
+               for n, r in (("one-rank parallel", y1), ("serial", ys)) if not torch.equal(y, r)]
+        q.put((rank, "ok" if not bad and y.dtype == torch.float32 else f"MISMATCH ({y.dtype}): {bad}"))
     except Exception as e:  # noqa
         q.put((rank, f"FAIL {type(e).__name__}: {e}"))
     finally:
